@@ -33,6 +33,9 @@ inside it.
               all-gathered checksum against both eyes computed on one GPU
   --impl reference : the CPU reference arm (same metric / config), rank 0 only under torchrun; a step = one stereo
               pair (a bounded sample of the 256-pair step)
+  --dump-outputs DIR : after the timed steps, rank 0 writes the eye textures its last step handed back as
+              DIR/frame<i>_<eye>.npy (float32 texel codes at a fixed, seeded sample of pixels), so that two builds can be
+              compared output for output on the same inputs
 
 Multi-GPU: frames are independent (SURVEY.md 8e) -> each rank processes its own pool, no data-path
 collective; NCCL only broadcasts the constant block from rank 0 and forms the barriers.  scaling = weak.
@@ -264,7 +267,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline + roofline only")
     ap.add_argument("--no-ncu", action="store_true", help="skip the ncu child that measures DRAM traffic / instructions")
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)  # the ncu child's workload
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last step as DIR/<name>.npy (float32, sampled)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -341,6 +350,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     pairs = world * PAIRS_PER_STEP * args.steps
     value = pairs / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(runner, args.dump_outputs)
     runner.close()
 
     # ---- instrumented pass: per-kernel CUDA events on the launch stream (roofline of the dominant kernel)
@@ -492,6 +503,7 @@ class EyeStreams:
 
     def __init__(self, ovr, torch, cfg, dev, n_streams, pair=False):
         self.pair = pair  # one caller stream, both eyes handed over in one PostProcessor.apply_pair call
+        self.last = {}  # context -> (pool index, (left out, right out)) of the last frame it processed
         self.main = torch.cuda.current_stream(dev)
         self.pps = [ovr.PostProcessor(cfg) for _ in range(max(1, n_streams // 2))]
         if n_streams == 1:
@@ -504,10 +516,12 @@ class EyeStreams:
         for i in (range(len(pool)) if frames is None else frames):
             left, right = pool[i % len(pool)]
             if self.pair:
-                self.pps[i % n].apply_pair(left, right, stream=self.streams[i % n][0])
-                continue
-            self.pps[i % n].apply(0, left, stream=self.streams[i % n][0])
-            self.pps[i % n].apply(1, right, stream=self.streams[i % n][1])
+                outs = self.pps[i % n].apply_pair(left, right, stream=self.streams[i % n][0])
+            else:
+                outs = (self.pps[i % n].apply(0, left, stream=self.streams[i % n][0]),
+                        self.pps[i % n].apply(1, right, stream=self.streams[i % n][1]))
+            # the returned views stay valid until the context's next apply of the same eye
+            self.last[i % n] = (i % len(pool), outs)
 
     def fork(self):
         for pair in self.streams:
@@ -524,6 +538,25 @@ class EyeStreams:
     def close(self):
         for p in self.pps:
             p.close()
+
+
+DUMP_PIXELS = 1 << 18  # 4 MiB of float32 per eye texture; --streams 8 leaves 8 of them: 32 MiB in all
+
+
+def dump_outputs(runner, directory):
+    """--dump-outputs: the eye textures the last step handed back that the contexts still hold (the last frame each
+    context processed, both eyes; the earlier frames' outputs were overwritten inside the step), once the step has
+    finished.  A 2244x2492 RGBA8 eye is 89 MB as float32, so each file holds the texel codes of the same DUMP_PIXELS
+    pixels, drawn without replacement with seed 0 and sorted (row-major index): shape (DUMP_PIXELS, 4)."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    idx = None
+    for frame, eyes in sorted(runner.last.values(), key=lambda fe: fe[0]):
+        for name, t in zip(("left", "right"), eyes):
+            px = t.contiguous().cpu().numpy().reshape(-1, 4)
+            if idx is None:
+                idx = np.sort(np.random.default_rng(0).choice(px.shape[0], DUMP_PIXELS, replace=False))
+            np.save(out / f"frame{frame}_{name}.npy", px[idx].astype(np.float32))
 
 
 def quick_value(ovr, torch, cfg, pool, passes, n_streams, pair=False):

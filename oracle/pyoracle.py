@@ -70,7 +70,11 @@ def build(force: bool = False) -> None:
         subprocess.check_call(["make", "-C", str(HERE), "libovrfsr_oracle.so"], stdout=subprocess.DEVNULL)
     ref_root = Path(os.environ.get("OVRFSR_REFERENCE", "/root/reference"))
     ref_so = HERE / "_ref" / "libovrfsr_ref.so"
-    if (ref_root / "src/fsr/ffx_fsr1.h").exists():
+    try:
+        have_ref = (ref_root / "src/fsr/ffx_fsr1.h").exists()
+    except OSError:  # a parent directory this user may not search: the sources are not available to it
+        have_ref = False
+    if have_ref:
         shim = list((HERE / "ref_shim").glob("*.cpp")) + [HERE / "build_ref.sh", HERE / "ovr_glue.h",
                                                            HERE / "fsr_entry.inc"]
         if force or not ref_so.exists() or any(p.stat().st_mtime > ref_so.stat().st_mtime for p in shim if p.exists()):

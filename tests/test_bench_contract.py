@@ -1,6 +1,7 @@
 """bench.py's command-line contract, as far as a box without a GPU can check it: the reference arm (the reference's own
 lines on the host cores) prints ONE JSON line with the keys the driver reads, on the same config object as the product
-arm; the product arm refuses to run without a CUDA device instead of falling back to anything."""
+arm; the product arm refuses to run without a CUDA device instead of falling back to anything.  On a GPU:
+--dump-outputs writes what the timed path computed."""
 import json
 import subprocess
 import sys
@@ -17,8 +18,6 @@ def _run(*args, timeout=600):
 
 def test_reference_arm_prints_the_contract_line():
     from oracle import pyoracle as po
-    if not po.ref_available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
     r = _run("--impl", "reference", "--steps", "1", "--warmup", "0")
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
@@ -30,9 +29,41 @@ def test_reference_arm_prints_the_contract_line():
     assert d["scaling"] == "weak" and d["vs_baseline"] is None and d["dtype"] == "f32" and d["data"] == "synthetic"
     assert d["config"]["workload"].startswith("C2: stereo 1683x1869->2244x2492") and d["config"]["radius"] == 2.0
     cb = d["cpu_baseline"]
-    assert cb["kind"] == "reference" and cb["cores"] >= 1 and cb["value"] == d["value"] and "pair" in cb["sample"]
+    # without the original's sources (no oracle/_ref) the arm runs the restated oracle and says so
+    assert cb["kind"] == ("reference" if po.ref_available() else "port") and cb["cores"] >= 1 and cb["value"] == d["value"] and "pair" in cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["gpu_launches"] == 0  # nothing of the product runs on this arm
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_steps_outputs(cuda, tmp_path):
+    """--dump-outputs: float32 samples, within 64 MB, of the eye textures the last timed step handed back (the last
+    frame of each of the 2 contexts at --streams 4), equal to the oracle's EASU+RCAS of the same pool frames."""
+    import os
+
+    import numpy as np
+
+    import bench
+    from openvr_fsr_b200 import synth
+    from oracle import pyoracle as po
+    r = _run("--steps", "2", "--no-extras", "--no-e2e", "--no-cpu-baseline", "--no-ncu", "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])["steps"] == 2
+    files = sorted(tmp_path.glob("*.npy"))
+    assert {f.stem for f in files} == {f"frame{bench.POOL - k}_{e}" for k in (1, 2) for e in ("left", "right")}
+    assert sum(f.stat().st_size for f in files) <= 64 << 20
+    base = synth.stereo_pair("natural", bench.IN_W, bench.IN_H, 1)
+    idx = np.sort(np.random.default_rng(0).choice(bench.OUT_W * bench.OUT_H, bench.DUMP_PIXELS, replace=False))
+    for f in files:
+        frame, eye = int(f.stem.split("_")[0][5:]), ("left", "right").index(f.stem.split("_")[1])
+        got = np.load(f)
+        assert got.dtype == np.float32 and got.shape == (bench.DUMP_PIXELS, 4)
+        src = np.roll(base[eye], 37 * frame, axis=0)  # bench.build_pool's frame of rank 0
+        uc = po.upscale_constants(eye, True, bench.IN_W, bench.IN_H, bench.OUT_W, bench.OUT_H, radius=2.0)
+        sc = po.sharpen_constants(eye, True, bench.OUT_W, bench.OUT_H, radius=2.0, sharpness=bench.SHARPNESS)
+        n = os.cpu_count() or 1
+        want = po.rcas(po.easu(src, bench.OUT_W, bench.OUT_H, uc, nthreads=n), sc, nthreads=n)
+        assert np.array_equal(got, want.reshape(-1, 4)[idx].astype(np.float32)), f.name
 
 
 def test_product_arm_fails_loudly_without_a_gpu():

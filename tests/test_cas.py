@@ -1,12 +1,14 @@
 """Legacy CAS path (src/cas, SURVEY 8f row 4): the restated oracle against the reference's own CasSetup / CasFilter
 lines compiled on the host (oracle/_ref), bit for bit."""
+from pathlib import Path
+
 import numpy as np
 import pytest
 
 from oracle import pyoracle as po
 from openvr_fsr_b200 import synth
 
-needs_ref = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (no /root/reference here)")
+needs_ref = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built: the original project's sources are absent")
 
 
 @needs_ref
@@ -17,6 +19,18 @@ def test_cas_setup_matches_reference(sharp, mcd):
         a = po.cas_setup(sharp, mcd, iw, ih, ow, oh)
         b = po.cas_setup(sharp, mcd, iw, ih, ow, oh, which="ref")
         assert np.array_equal(a.words(), b.words()), (sharp, mcd, iw, ih, a.words(), b.words())
+
+
+@pytest.mark.parametrize("name,sharp,mcd", [("sharpen_natural_57x41", 0.8, 1.0), ("sharpen_clamped_57x41", 1.0, 0.06),
+                                            ("upscale_natural_57x41_s067", 0.9, 1.0), ("upscale_fp16_33x27_s05", 0.5, 1.0)])
+def test_cas_setup_matches_golden(name, sharp, mcd):
+    """The words the reference's own CasSetup produced for the pass_cas_* fixtures (tests/golden/make_golden_more.py),
+    checked where the reference's sources are absent: the oracle's and the library's CasSetup must reproduce them."""
+    import openvr_fsr_b200 as ovr
+    g = np.load(Path(__file__).parent / "golden" / f"pass_cas_{name}.npz")
+    (ih, iw), (oh, ow) = g["src"].shape[:2], g["out"].shape[:2]
+    assert np.array_equal(po.cas_setup(sharp, mcd, iw, ih, ow, oh).words(), g["consts"])
+    assert np.array_equal(ovr.cas_setup(sharp, mcd, iw, ih, ow, oh), g["consts"])
 
 
 @needs_ref

@@ -71,7 +71,7 @@ def test_rcas_con_sweep_matches_oracle():
         assert list(a) == list(b)
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built")
+@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built: the original project's sources are absent")
 def test_constants_match_reference_functions():
     lib, ref = L.lib(), po.ref_lib()
     rng = np.random.default_rng(11)

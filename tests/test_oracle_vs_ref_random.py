@@ -7,7 +7,7 @@ import pytest
 from oracle import pyoracle as po
 from openvr_fsr_b200 import synth
 
-pytestmark = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (no /root/reference here)")
+pytestmark = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built: the original project's sources are absent")
 
 
 def _image(rng, w, h, fmt):
