@@ -170,6 +170,44 @@ OVRFSR_API int ovrfsr_apply_host(ovrfsr_ctx *ctx, int eye, const ovrfsr_image *s
 OVRFSR_API int ovrfsr_apply_pair(ovrfsr_ctx *ctx, const ovrfsr_image *src_left, const ovrfsr_image *src_right,
                                  int only_one_eye, ovrfsr_image out[2], void *stream);
 
+/* VRTextureBounds_t (headers/openvr.h:609-613): the part of an eye texture that holds the image, in [0, 1] texture
+ * coordinates.  {0, 0, 1, 1} is the whole texture. */
+typedef struct ovrfsr_bounds {
+  float u_min, v_min, u_max, v_max;
+} ovrfsr_bounds;
+/* a rectangle of texels: x, y = its top-left texel */
+typedef struct ovrfsr_rect {
+  uint32_t x, y, width, height;
+} ovrfsr_rect;
+
+/* Extension: ovrfsr_apply for an eye submitted with texture bounds (dynamic resolution, both eyes side by side in one
+ * texture).  The eye is processed exactly as if its rectangle had been cut out as a texture of its own and given to
+ * ovrfsr_apply with only_one_eye = 1, and the result is written at the matching rectangle of the usual full-size
+ * output, so the compositor's bounds still address the output unchanged:
+ *   - rectangles (single-precision host arithmetic): u0 = clamp(min(u_min, u_max), 0, 1), u1 = clamp(max(u_min, u_max),
+ *     0, 1), likewise v (flipped bounds give the same rectangle; the flip stays with the compositor);
+ *     source x0 = (uint32_t)(u0 * (float)W + 0.5f), x1 = (uint32_t)(u1 * (float)W + 0.5f), likewise y with H, in the
+ *     eye's texture (its slice for an array texture) of W x H texels; the output rectangle is the same formula on the
+ *     ctx output size ovrfsr_output_size(W, H, renderScale).  ovrfsr_bounds_rects computes both.
+ *   - constants: ovrfsr_make_upscale_constants / _sharpen_constants / ovrfsr_make_nis_config for the eye with the
+ *     rectangle sizes and only_one_eye = 1 -- the foveation centre and radius follow the view;
+ *   - at the rectangle's edges EASU, NVScaler and NVSharpen clamp to the edge and RCAS reads zero, as at a texture's
+ *     edge; texels outside the source rectangle never influence the result, pixels outside the output rectangle are
+ *     not written.
+ * Each call processes its eye (no "shared texture processed once" rule: a side-by-side texture is two rectangles).  A
+ * rectangle change is not a size change: it resets, reallocates and synchronises nothing; a texture size or format
+ * change resets as in ovrfsr_apply.  ovrfsr_apply and ovrfsr_apply_bounds may be mixed on one ctx.  The opt-in fused
+ * kernel (OVRFSR_FLAG_FUSED_FSR) runs only for full bounds; other rectangles take the two dispatches (same bits).
+ *   bounds    NULL = {0, 0, 1, 1}; an empty rectangle (either dimension) is OVRFSR_ERR_INVALID
+ *   out       the full ctx-owned output image, as ovrfsr_apply returns it
+ *   out_rect  nullable: receives the output rectangle */
+OVRFSR_API int ovrfsr_apply_bounds(ovrfsr_ctx *ctx, int eye, const ovrfsr_image *src, const ovrfsr_bounds *bounds,
+                                   ovrfsr_image *out, ovrfsr_rect *out_rect, void *stream);
+/* The two rectangles of ovrfsr_apply_bounds for a W x H eye texture and an out_w x out_h output (pure CPU).  bounds NULL
+ * = {0, 0, 1, 1}.  OVRFSR_ERR_INVALID for an empty rectangle or NaN bounds; either output pointer may be NULL. */
+OVRFSR_API int ovrfsr_bounds_rects(uint32_t w, uint32_t h, uint32_t out_w, uint32_t out_h, const ovrfsr_bounds *bounds,
+                                   ovrfsr_rect *src_rect, ovrfsr_rect *dst_rect);
+
 /* ---- individual dispatches (ApplyUpscaling / ApplySharpening, PostProcessor.cpp:385-401,483-496) --
  * Stateless: explicit constant blocks, caller-owned destination.  math_mode as ovrfsr_math. */
 /* g_FSRUpscaleShader: consts = UpscaleConstants, 24 x u32 (PostProcessor.cpp:276-283) */

@@ -9,4 +9,4 @@ from ._lib import (ERR_CUDA, ERR_INVALID, ERR_NOMEM, ERR_UNSUPPORTED, FORMAT_AUT
 from .api import (EYE_LEFT, EYE_RIGHT, Config, PostProcessor, TextureBounds, alloc_image, fsr_easu, fsr_fused, fsr_rcas, image_of,  # noqa
                   kernel_launches, make_nis_config, make_sharpen_constants, make_upscale_constants, nis_scaler,
                   nis_sharpen, output_size, to_image, resolve_msaa, expand_rgb32f, format_considered_srgb, recommended_render_size, mip_lod_bias,
-                  sampler_lod_bias, capture_filename, save_dds, load_dds, cas, cas_setup)
+                  sampler_lod_bias, capture_filename, save_dds, load_dds, cas, cas_setup, bounds_rects)

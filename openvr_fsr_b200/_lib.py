@@ -25,6 +25,14 @@ class Image(C.Structure):
                 ("sample_count", C.c_uint32)]
 
 
+class Bounds(C.Structure):
+    _fields_ = [("u_min", C.c_float), ("v_min", C.c_float), ("u_max", C.c_float), ("v_max", C.c_float)]
+
+
+class Rect(C.Structure):
+    _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("width", C.c_uint32), ("height", C.c_uint32)]
+
+
 class Config(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("fsr_enabled", C.c_int32), ("use_nis", C.c_int32),
                 ("render_scale", C.c_float), ("sharpness", C.c_float), ("radius", C.c_float),
@@ -44,6 +52,8 @@ SYMBOLS = {
     "ovrfsr_apply": (C.c_int, [_vp, C.c_int, _imgp, C.c_int, _imgp, _vp]),
     "ovrfsr_apply_host": (C.c_int, [_vp, C.c_int, _imgp, C.c_int, _imgp, _vp]),
     "ovrfsr_apply_pair": (C.c_int, [_vp, _imgp, _imgp, C.c_int, _imgp, _vp]),
+    "ovrfsr_apply_bounds": (C.c_int, [_vp, C.c_int, _imgp, C.POINTER(Bounds), _imgp, C.POINTER(Rect), _vp]),
+    "ovrfsr_bounds_rects": (C.c_int, [C.c_uint32] * 4 + [C.POINTER(Bounds), C.POINTER(Rect), C.POINTER(Rect)]),
     "ovrfsr_dispatch_fsr_easu": (C.c_int, [_imgp, _imgp, _u32p, C.c_int, _vp]),
     "ovrfsr_dispatch_fsr_rcas": (C.c_int, [_imgp, _imgp, _u32p, C.c_int, _vp]),
     "ovrfsr_dispatch_fsr_fused": (C.c_int, [_imgp, _imgp, _u32p, _u32p, C.c_int, _vp]),

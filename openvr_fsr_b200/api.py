@@ -176,6 +176,22 @@ class PostProcessor:
         self.last_output_format = outs[0].format
         return _wrap_device(outs[0], left.device), _wrap_device(outs[1], right.device)
 
+    def apply_bounds(self, eye: int, texture, bounds: TextureBounds | None = None, fmt: int | None = None, stream=None,
+                     samples: int = 1):
+        """ovrfsr_apply_bounds: post-process only the `bounds` rectangle of the eye texture, as if it had been cut out
+        as a texture of its own, and write the result at the matching rectangle of the full-size output.  Returns
+        (output view, (x, y, w, h) of the output rectangle), or (`texture`, None) on pass-through."""
+        b = bounds or TextureBounds()
+        cb, rect = L.Bounds(b.uMin, b.vMin, b.uMax, b.vMax), L.Rect()
+        src, out = image_of(texture, fmt, samples), L.Image()
+        rc = L.lib().ovrfsr_apply_bounds(self._ctx, eye, C.byref(src), C.byref(cb), C.byref(out), C.byref(rect),
+                                         _stream_ptr(stream))
+        if rc == L.PASSTHROUGH:
+            return texture, None
+        L.check(rc, "ovrfsr_apply_bounds", self._ctx)
+        self.last_output_format = out.format
+        return _wrap_device(out, texture.device), (rect.x, rect.y, rect.width, rect.height)
+
     def apply_host(self, eye: int, src_host, dst_host, bounds: TextureBounds | None = None, fmt: int | None = None,
                    stream=None, dst_fmt: int | None = None):
         """End-to-end entry: host (pinned) tensors in and out, copies included, asynchronous on `stream`."""
@@ -342,6 +358,16 @@ def load_dds(path: str) -> tuple[np.ndarray, int]:
         return raw.view(dt).reshape(img.height, img.width, 4), img.format
     finally:
         L.lib().ovrfsr_host_free(img.data)
+
+
+def bounds_rects(width: int, height: int, out_w: int, out_h: int, bounds: TextureBounds | None = None):
+    """The source and output rectangles ovrfsr_apply_bounds uses, each (x, y, w, h); raises OvrFsrError
+    (ERR_INVALID) for an empty rectangle."""
+    b = bounds or TextureBounds()
+    cb, s, d = L.Bounds(b.uMin, b.vMin, b.uMax, b.vMax), L.Rect(), L.Rect()
+    L.check(L.lib().ovrfsr_bounds_rects(width, height, out_w, out_h, C.byref(cb), C.byref(s), C.byref(d)),
+            "ovrfsr_bounds_rects")
+    return (s.x, s.y, s.width, s.height), (d.x, d.y, d.width, d.height)
 
 
 def make_upscale_constants(cfg: Config, eye, only_one_eye, in_w, in_h, out_w, out_h) -> np.ndarray:

@@ -5,6 +5,7 @@
 #include <atomic>
 #include <cstdio>
 #include <cstdlib>
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <ctime>
@@ -110,6 +111,24 @@ PassImage pass_image(const ovrfsr_image &im, int slice = 0) {
   p.pitch = im.pitch; p.w = (int)im.width; p.h = (int)im.height; p.format = im.format;
   return p;
 }
+// the rectangle r of the whole image t (nullptr: all of it)
+PassImage crop(const PassImage &t, const ovrfsr_rect *r) {
+  if (!r) return t;
+  PassImage p = t;
+  p.ptr = static_cast<uint8_t *>(t.ptr) + (size_t)r->y * t.pitch + (size_t)r->x * bytes_per_pixel(t.format);
+  p.w = (int)r->width; p.h = (int)r->height;
+  p.x0 = (int)r->x; p.y0 = (int)r->y; p.texW = t.w; p.texH = t.h;
+  return p;
+}
+inline bool same_rect(const ovrfsr_rect &a, const ovrfsr_rect &b) {
+  return a.x == b.x && a.y == b.y && a.width == b.width && a.height == b.height;
+}
+
+// the constant blocks one apply runs with
+struct EyeConsts {
+  const uint32_t *upscale, *sharpen;
+  const uint8_t *nisScaler, *nisSharpen;
+};
 
 } // namespace
 
@@ -127,6 +146,14 @@ struct ovrfsr_ctx {
   uint32_t sharpenConstants[2][12]{};
   alignas(16) uint8_t nisScalerConfig[2][256]{};
   alignas(16) uint8_t nisSharpenConfig[2][256]{};
+  // ovrfsr_apply_bounds: per eye, the last rectangles and the constant blocks built for them (beside the full-texture
+  // ones above, so that ovrfsr_apply and ovrfsr_apply_bounds can be mixed on one ctx)
+  struct BoundsEye {
+    bool valid = false;
+    ovrfsr_rect src{}, dst{};
+    uint32_t upscale[24]{}, sharpen[12]{};
+    alignas(16) uint8_t nisScaler[256]{}, nisSharpen[256]{};
+  } bounds[2];
   // one set of intermediates/outputs PER EYE (the reference shares one; see ovrfsr.h)
   DeviceImage upscaled[2], sharpened[2];
   DeviceImage hostStage[2]; // device staging of host-submitted eyes (ovrfsr_apply_host)
@@ -249,34 +276,34 @@ bool paired_passes(const ovrfsr_ctx *c) {
          (c->outFormat == OVRFSR_FORMAT_RGBA8 || c->outFormat == OVRFSR_FORMAT_RGB10A2);
 }
 
-int run_upscale(ovrfsr_ctx *c, int eye, const PassImage &in, const PassImage &out, cudaStream_t s) {
+int nis_status(cudaError_t e) {
+  if (e == cudaSuccess) return OVRFSR_OK;
+  return (e == cudaErrorInvalidConfiguration || e == cudaErrorInvalidValue) ? OVRFSR_ERR_UNSUPPORTED : OVRFSR_ERR_CUDA;
+}
+
+// `fin` = the final image (the output rectangle of the sharpened texture): the paired EASU writes its outside-radius
+// groups there
+int run_upscale(ovrfsr_ctx *c, const EyeConsts &k, const PassImage &in, const PassImage &out, const PassImage &fin, cudaStream_t s) {
   const bool strict = c->cfg.math_mode == OVRFSR_MATH_STRICT;
   cudaError_t e;
   if (c->cfg.use_nis) {
-    ovrfsr_image si{in.ptr, (uint32_t)in.w, (uint32_t)in.h, in.pitch, in.format, 1, 0};
-    ovrfsr_image di{out.ptr, (uint32_t)out.w, (uint32_t)out.h, out.pitch, out.format, 1, 0};
-    int rc = ovrfsr_dispatch_nis_scaler(&si, &di, c->nisScalerConfig[eye], c->cfg.math_mode, s);
+    int rc = nis_status(launch_nis(false, in, out, k.nisScaler, c->cfg.math_mode, s));
     return rc == OVRFSR_OK ? rc : fail(c, rc, "NIS scaler dispatch");
   }
-  const PassImage fin = pass_image(c->sharpened[eye].img);
   const PassImage *direct = paired_passes(c) ? &fin : nullptr;
-  const float tint = 1.0f - (float)c->sharpenConstants[eye][3] * 0.3f;
-  e = strict ? launch_easu_strict(in, out, c->upscaleConstants[eye], s, direct, tint)
-             : launch_easu_fast(in, out, c->upscaleConstants[eye], s, direct, tint);
+  const float tint = 1.0f - (float)k.sharpen[3] * 0.3f;
+  e = strict ? launch_easu_strict(in, out, k.upscale, s, direct, tint) : launch_easu_fast(in, out, k.upscale, s, direct, tint);
   return e == cudaSuccess ? OVRFSR_OK : fail(c, OVRFSR_ERR_CUDA, "EASU launch", e);
 }
 
-int run_sharpen(ovrfsr_ctx *c, int eye, const PassImage &in, const PassImage &out, cudaStream_t s) {
+int run_sharpen(ovrfsr_ctx *c, const EyeConsts &k, const PassImage &in, const PassImage &out, cudaStream_t s) {
   const bool strict = c->cfg.math_mode == OVRFSR_MATH_STRICT;
   if (c->cfg.use_nis) {
-    ovrfsr_image si{in.ptr, (uint32_t)in.w, (uint32_t)in.h, in.pitch, in.format, 1, 0};
-    ovrfsr_image di{out.ptr, (uint32_t)out.w, (uint32_t)out.h, out.pitch, out.format, 1, 0};
-    int rc = ovrfsr_dispatch_nis_sharpen(&si, &di, c->nisSharpenConfig[eye], c->cfg.math_mode, s);
+    int rc = nis_status(launch_nis(true, in, out, k.nisSharpen, c->cfg.math_mode, s));
     return rc == OVRFSR_OK ? rc : fail(c, rc, "NIS sharpen dispatch");
   }
   const bool skip = paired_passes(c);
-  cudaError_t e = strict ? launch_rcas_strict(in, out, c->sharpenConstants[eye], s, skip)
-                         : launch_rcas_fast(in, out, c->sharpenConstants[eye], s, skip);
+  cudaError_t e = strict ? launch_rcas_strict(in, out, k.sharpen, s, skip) : launch_rcas_fast(in, out, k.sharpen, s, skip);
   return e == cudaSuccess ? OVRFSR_OK : fail(c, OVRFSR_ERR_CUDA, "RCAS launch", e);
 }
 
@@ -298,8 +325,12 @@ int save_capture(ovrfsr_ctx *c, const ovrfsr_image &img, cudaStream_t s) {
 }
 
 // PostProcessor::ApplyPostProcess, PostProcessor.cpp:563-638 (the D3D11 binding save/restore and the Win32 hotkey
-// polling stay in the caller; the F7 capture is served through ovrfsr_request_capture)
-int apply_post_process(ovrfsr_ctx *c, int eye, const ovrfsr_image *src, ovrfsr_image *out, cudaStream_t s) {
+// polling stay in the caller; the F7 capture is served through ovrfsr_request_capture).
+// srcRect / dstRect (ovrfsr_apply_bounds, nullptr = the whole images): the passes read the source rectangle of the
+// (resolved / expanded / sliced) eye texture and write the output rectangle of the ctx images; `k` holds the constants
+// built for those sizes.
+int apply_post_process(ovrfsr_ctx *c, int eye, const ovrfsr_image *src, ovrfsr_image *out, cudaStream_t s, const EyeConsts &k,
+                       const ovrfsr_rect *srcRect = nullptr, const ovrfsr_rect *dstRect = nullptr) {
   // GetInputView: array textures keep the right eye in slice 1 (PostProcessor.cpp:254-268)
   const int slice = (src->array_slices > 1 && eye == 1) ? 1 : 0;
   PassImage in = pass_image(*src, slice);
@@ -326,6 +357,7 @@ int apply_post_process(ovrfsr_ctx *c, int eye, const ovrfsr_image *src, ovrfsr_i
     in = pass_image(x.img);
     result = x.img;
   }
+  in = crop(in, srcRect);
   int q = -1;
   if (c->evCreated) {
     harvest_queries(c);
@@ -339,22 +371,22 @@ int apply_post_process(ovrfsr_ctx *c, int eye, const ovrfsr_image *src, ovrfsr_i
     // ApplyUpscaling + ApplySharpening (PostProcessor.cpp:586-594) as one kernel; shapes it does not cover take the
     // two dispatches below
     const bool strict = c->cfg.math_mode == OVRFSR_MATH_STRICT;
-    const PassImage out2 = pass_image(c->sharpened[eye].img);
-    const cudaError_t e = strict ? launch_fsr_fused_strict(in, out2, c->upscaleConstants[eye], c->sharpenConstants[eye], s)
-                                 : launch_fsr_fused_fast(in, out2, c->upscaleConstants[eye], c->sharpenConstants[eye], s);
+    const PassImage out2 = crop(pass_image(c->sharpened[eye].img), dstRect);
+    const cudaError_t e = strict ? launch_fsr_fused_strict(in, out2, k.upscale, k.sharpen, s) : launch_fsr_fused_fast(in, out2, k.upscale, k.sharpen, s);
     if (e == cudaSuccess) { fused = true; result = c->sharpened[eye].img; }
     else if (e != cudaErrorInvalidValue && e != cudaErrorInvalidConfiguration) return fail(c, OVRFSR_ERR_CUDA, "fused EASU+RCAS launch", e);
   }
   if (!fused && upscale_pass(c->cfg)) {
     if (!c->upscaled[eye].img.data && !c->upscaled[eye].alloc(c->outputWidth, c->outputHeight, c->outFormat))
       return fail(c, OVRFSR_ERR_NOMEM, "allocating upscaled texture", cudaGetLastError());
-    int rc = run_upscale(c, eye, in, pass_image(c->upscaled[eye].img), s);
+    const PassImage mid = crop(pass_image(c->upscaled[eye].img), dstRect);
+    int rc = run_upscale(c, k, in, mid, crop(pass_image(c->sharpened[eye].img), dstRect), s);
     if (rc != OVRFSR_OK) return rc;
-    in = pass_image(c->upscaled[eye].img);
+    in = mid;
     result = c->upscaled[eye].img;
   }
   if (!fused && sharpen_pass(c->cfg)) {
-    int rc = run_sharpen(c, eye, in, pass_image(c->sharpened[eye].img), s);
+    int rc = run_sharpen(c, k, in, crop(pass_image(c->sharpened[eye].img), dstRect), s);
     if (rc != OVRFSR_OK) return rc;
     result = c->sharpened[eye].img;
   }
@@ -433,6 +465,7 @@ int ovrfsr_reset(ovrfsr_ctx *ctx) {
   }
   ctx->enabled = true;
   ctx->initialized = false;
+  ctx->bounds[0].valid = ctx->bounds[1].valid = false;
   ctx->lastSubmittedTexture = nullptr;
   ctx->lastOutput = ovrfsr_image{};
   ctx->eyeCount = 0;
@@ -479,13 +512,79 @@ int ovrfsr_apply(ovrfsr_ctx *ctx, int eye, const ovrfsr_image *src_tagged, int o
   }
   // a single shared texture for both eyes is processed on the first Submit only (PostProcessor.cpp:155-160)
   if (ctx->eyeCount == 0 || ctx->textureContainsOnlyOneEye || src->data != ctx->lastSubmittedTexture) {
-    rc = apply_post_process(ctx, ctx->textureContainsOnlyOneEye ? eye : 0, src, &ctx->lastOutput,
-                            static_cast<cudaStream_t>(stream));
+    const int e = ctx->textureContainsOnlyOneEye ? eye : 0;
+    const EyeConsts k{ctx->upscaleConstants[e], ctx->sharpenConstants[e], ctx->nisScalerConfig[e], ctx->nisSharpenConfig[e]};
+    rc = apply_post_process(ctx, e, src, &ctx->lastOutput, static_cast<cudaStream_t>(stream), k);
     if (rc != OVRFSR_OK) return rc;
   }
   ctx->lastSubmittedTexture = src->data;
   ctx->eyeCount = (ctx->eyeCount + 1) % 2;
   *out = ctx->lastOutput;
+  return OVRFSR_OK;
+}
+
+int ovrfsr_bounds_rects(uint32_t w, uint32_t h, uint32_t out_w, uint32_t out_h, const ovrfsr_bounds *bounds,
+                        ovrfsr_rect *src_rect, ovrfsr_rect *dst_rect) {
+  const ovrfsr_bounds whole{0.f, 0.f, 1.f, 1.f};
+  const ovrfsr_bounds &b = bounds ? *bounds : whole;
+  if (std::isnan(b.u_min) || std::isnan(b.v_min) || std::isnan(b.u_max) || std::isnan(b.v_max)) return OVRFSR_ERR_INVALID;
+  const auto unit = [](float t) { return t < 0.f ? 0.f : (t > 1.f ? 1.f : t); };
+  const float u0 = unit(std::fmin(b.u_min, b.u_max)), u1 = unit(std::fmax(b.u_min, b.u_max));
+  const float v0 = unit(std::fmin(b.v_min, b.v_max)), v1 = unit(std::fmax(b.v_min, b.v_max));
+  const auto edge = [](float t, uint32_t n) {
+    const float p = t * (float)n;
+    return (uint32_t)(p + 0.5f);
+  };
+  const ovrfsr_rect s{edge(u0, w), edge(v0, h), edge(u1, w) - edge(u0, w), edge(v1, h) - edge(v0, h)};
+  const ovrfsr_rect d{edge(u0, out_w), edge(v0, out_h), edge(u1, out_w) - edge(u0, out_w), edge(v1, out_h) - edge(v0, out_h)};
+  if (s.width == 0 || s.height == 0 || d.width == 0 || d.height == 0) return OVRFSR_ERR_INVALID;
+  if (src_rect) *src_rect = s;
+  if (dst_rect) *dst_rect = d;
+  return OVRFSR_OK;
+}
+
+int ovrfsr_apply_bounds(ovrfsr_ctx *ctx, int eye, const ovrfsr_image *src_tagged, const ovrfsr_bounds *bounds, ovrfsr_image *out,
+                        ovrfsr_rect *out_rect, void *stream) {
+  if (!ctx || !out || (eye != 0 && eye != 1)) return OVRFSR_ERR_INVALID;
+  ovrfsr_image src_untagged{};
+  if (src_tagged) src_untagged = untagged(src_tagged);
+  const ovrfsr_image *src = src_tagged ? &src_untagged : nullptr;
+  if (!ctx->enabled || !ctx->cfg.fsr_enabled) return OVRFSR_PASSTHROUGH;
+  int rc = validate_image(src);
+  if (rc != OVRFSR_OK) return fail(ctx, rc, "invalid source image");
+  if ((rc = select_device(ctx)) != OVRFSR_OK) return rc;
+  if (ctx->initialized && (src->width != ctx->inputWidth || src->height != ctx->inputHeight || src->format != ctx->inFormat))
+    ovrfsr_reset(ctx); // a texture size or format change, as in ovrfsr_apply (a rectangle change is not one)
+  if (!ctx->initialized) {
+    ctx->textureContainsOnlyOneEye = true;
+    rc = prepare_resources(ctx, src);
+    if (rc != OVRFSR_OK) {
+      release_resources(ctx);
+      ctx->enabled = false;
+      return rc;
+    }
+  }
+  ovrfsr_rect sr, dr;
+  if ((rc = ovrfsr_bounds_rects(src->width, src->height, ctx->outputWidth, ctx->outputHeight, bounds, &sr, &dr)) != OVRFSR_OK)
+    return fail(ctx, rc, "texture bounds select an empty rectangle");
+  ovrfsr_ctx::BoundsEye &b = ctx->bounds[eye];
+  if (!b.valid || !same_rect(b.src, sr) || !same_rect(b.dst, dr)) {
+    host::make_upscale_constants(b.upscale, ctx->cfg, eye, true, sr.width, sr.height, dr.width, dr.height);
+    host::make_sharpen_constants(b.sharpen, ctx->cfg, eye, true, dr.width, dr.height);
+    ovrfsr_make_nis_config(b.nisScaler, &ctx->cfg, 0, eye, 1, sr.width, sr.height, dr.width, dr.height);
+    ovrfsr_make_nis_config(b.nisSharpen, &ctx->cfg, 1, eye, 1, sr.width, sr.height, dr.width, dr.height);
+    b.src = sr; b.dst = dr; b.valid = true;
+  }
+  // a ctx that ovrfsr_apply set up for one texture holding both eyes has no right-eye output yet
+  if (sharpen_pass(ctx->cfg) && !ctx->sharpened[eye].img.data &&
+      !ctx->sharpened[eye].alloc(ctx->outputWidth, ctx->outputHeight, ctx->outFormat))
+    return fail(ctx, OVRFSR_ERR_NOMEM, "allocating sharpened texture", cudaGetLastError());
+  const EyeConsts k{b.upscale, b.sharpen, b.nisScaler, b.nisSharpen};
+  ovrfsr_image result{};
+  rc = apply_post_process(ctx, eye, src, &result, static_cast<cudaStream_t>(stream), k, &sr, &dr);
+  if (rc != OVRFSR_OK) return rc;
+  *out = result;
+  if (out_rect) *out_rect = dr;
   return OVRFSR_OK;
 }
 

@@ -18,6 +18,9 @@ struct Config {
   int cudaDevice = -1;
   bool strictMath = true;   // bit-identical to the reference lines (the library default); false = FMA-contracted kernels, <= 1 LSB per pass
   bool fusedFsr = false;    // OVRFSR_FLAG_FUSED_FSR: one fused EASU->RCAS kernel instead of the two dispatches
+  // extension: post-process only the submitted VRTextureBounds_t rectangle of each eye (ovrfsr_apply_bounds) -- for
+  // dynamic resolution and side-by-side eyes.  false = the reference, which filters the whole texture.
+  bool honourTextureBounds = false;
 
   // ONE instance per process, owned by libovrfsr.so (an inline function-local static would be duplicated in every
   // module that includes this header when the library is built with hidden visibility)

@@ -40,6 +40,7 @@ struct EasuArgs {
   // intermediate `dst` only where an edge-adjacent group is inside the radius (RCAS reads one pixel across the edge).
   ImageRW direct;           // ptr == nullptr: plain dispatch
   float tintGB;             // 1 - debug*0.3 of the following RCAS pass
+  int x0, y0;               // src's origin in the texture srcMap describes (0, 0 unless src is a rectangle of it)
 };
 
 struct RcasArgs {
@@ -51,6 +52,11 @@ struct RcasArgs {
   uint32_t radiusSq;
   int skipOutside;          // the preceding EASU launch already wrote the outside-radius groups to dst (EasuArgs::direct)
   int opaqueSrc;            // B8G8R8X8 source: the X byte reads as alpha 1 (only the outside-radius copy looks at alpha)
+  // TMA variant: src is the rectangle at (x0, y0) of the texture srcMap describes.  Tile boxes start at x = ox0 + boxX
+  // (boxX = floor4(x0 - 1), a multiple of 4: the tile's first texel x0 - 1 lies boxShift = x0 - 1 - boxX texels into
+  // the box) and y = oy0 - 1 + y0.  zeroOutside: the rectangle is smaller than the texture, so the texels a box holds
+  // outside it are real data the kernel must replace by Texture2D.Load's out-of-bounds zero.
+  int y0, boxX, boxShift, zeroOutside;
 };
 
 // out pixel -> source position; the same instruction sequence is used for the tile origin and
@@ -389,7 +395,7 @@ __global__ void __launch_bounds__(kThreads, 3) easu_kernel(const __grid_constant
         int ox0, oy0, sx0, sy0;
         tile_origin(t, ox0, oy0, sx0, sy0);
         mbar_arrive_expect_tx(&tileBar, (uint32_t)(rawW * th * 4));
-        tma_load_2d(sRaw, &srcMap, sx0 & ~3, sy0, &tileBar); // box origin 16-byte aligned in x
+        tma_load_2d(sRaw, &srcMap, (sx0 + a.x0) & ~3, sy0 + a.y0, &tileBar); // box origin 16-byte aligned in x
       }
     }
     __syncthreads();
@@ -399,8 +405,9 @@ __global__ void __launch_bounds__(kThreads, 3) easu_kernel(const __grid_constant
   for (; t < numTiles; t += gridDim.x) {
     int ox0, oy0, sx0, sy0;
     tile_origin(t, ox0, oy0, sx0, sy0);
-    // float-tile origin and width in source texels: the TMA variant keeps the box's aligned origin
-    const int tx0 = TMA ? (sx0 & ~3) : sx0;
+    // float-tile origin and width in source texels: the TMA variant keeps the box's aligned origin (aligned in the
+    // texture, so within a rectangle at x0 % 4 != 0 it is up to 3 texels left of sx0)
+    const int tx0 = TMA ? ((sx0 + a.x0) & ~3) - a.x0 : sx0;
     const int cols = TMA ? rawW : a.tileW;
 
     // this warp's 16x16 group and its radius test (warp-uniform)
@@ -409,14 +416,15 @@ __global__ void __launch_bounds__(kThreads, 3) easu_kernel(const __grid_constant
 
     // ---- stage 1: decode the clamped source tile once, loads batched per thread for ILP -------------
     if constexpr (TMA) {
-      mbar_wait(&tileBar, phase); // this tile's box has landed (zeros outside the image)
+      mbar_wait(&tileBar, phase); // this tile's box has landed (zeros outside the texture)
       phase ^= 1u;
       const uint32_t *raw = sRaw;
 #pragma unroll
       for (int i = 0; i < kEasuColsPerThread; ++i) {
         const int tx = lane + 32 * i;
         if (tx < cols) {
-          const int rcol = clampi(tx0 + tx, 0, a.src.w - 1) - tx0; // clamp-to-edge: re-read the edge column / row
+          // clamp-to-edge: re-read the edge column / row of the image (of the rectangle: texels outside it are never used)
+          const int rcol = clampi(tx0 + tx, 0, a.src.w - 1) - tx0;
           uint32_t px[kEasuRowsPerThread];
 #pragma unroll
           for (int j = 0; j < kEasuRowsPerThread; ++j) {
@@ -460,7 +468,7 @@ __global__ void __launch_bounds__(kThreads, 3) easu_kernel(const __grid_constant
         tile_origin(tn2, nox, noy, nsx, nsy);
         fence_proxy_async();
         mbar_arrive_expect_tx(&tileBar, (uint32_t)(rawW * th * 4));
-        tma_load_2d(sRaw, &srcMap, nsx & ~3, nsy, &tileBar);
+        tma_load_2d(sRaw, &srcMap, (nsx + a.x0) & ~3, nsy + a.y0, &tileBar);
       }
     }
 
@@ -665,7 +673,7 @@ __global__ void __launch_bounds__(kThreads, 2) rcas_kernel(const __grid_constant
       mbar_init(&tileBar, 1);
       fence_barrier_init();
       mbar_arrive_expect_tx(&tileBar, (uint32_t)(kRcasTH * kRcasRawW * 4));
-      tma_load_2d(sRaw, &srcMap, ox0 - 4, sy0, &tileBar); // x origin 16-byte aligned: 3 unused texels on the left
+      tma_load_2d(sRaw, &srcMap, ox0 + a.boxX, sy0 + a.y0, &tileBar); // x origin 16-byte aligned: boxShift unused texels on the left
     }
   }
   const uint32_t ggx = blockIdx.x * (kTileW / 16) + (warp & 3), ggy = blockIdx.y * (kTileH / 16) + (warp >> 2);
@@ -678,14 +686,28 @@ __global__ void __launch_bounds__(kThreads, 2) rcas_kernel(const __grid_constant
     mbar_wait(&tileBar, 0);
     // the 34 x 66 texels as one flat index: 9 passes of the 256 threads, 97 % of the lanes busy (a row loop per warp with
     // a 32-wide column loop inside keeps 58 %: 66 columns take three column steps, 34 rows five row steps)
-    if (needTile)
+    // tile-uniform: the tile reaches over an edge of a rectangle that is smaller than the texture
+    const bool zeroEdge = a.zeroOutside && (sx0 < 0 || sy0 < 0 || sx0 + kTileW + 2 > a.src.w || sy0 + kRcasTH > a.src.h);
+    if (needTile && !zeroEdge) {
 #pragma unroll
       for (int q = tid; q < kRcasTH * (kTileW + 2); q += kThreads) {
         const int ty = q / (kTileW + 2), tx = q - ty * (kTileW + 2);
-        float4 c = decode_rgba<FIN>(sRaw[ty * kRcasRawW + tx + 3]);
+        float4 c = decode_rgba<FIN>(sRaw[ty * kRcasRawW + tx + a.boxShift]);
         if constexpr (OPQ) c.w = 1.0f;
         sC[ty * kRcasTW + tx] = c;
       }
+    } else if (needTile) {
+      for (int q = tid; q < kRcasTH * (kTileW + 2); q += kThreads) {
+        const int ty = q / (kTileW + 2), tx = q - ty * (kTileW + 2);
+        const int gy = sy0 + ty, gx = sx0 + tx;
+        float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (gy >= 0 && gy < a.src.h && gx >= 0 && gx < a.src.w) {
+          c = decode_rgba<FIN>(sRaw[ty * kRcasRawW + tx + a.boxShift]);
+          if constexpr (OPQ) c.w = 1.0f;
+        }
+        sC[ty * kRcasTW + tx] = c;
+      }
+    }
   } else {
     // Texture2D.Load semantics: out of bounds reads 0 (fsr_rcas.hlsl:18)
 #pragma unroll 3
@@ -723,7 +745,7 @@ __global__ void __launch_bounds__(kThreads, 2) rcas_kernel(const __grid_constant
       if (a.tintGB == 1.0f) {
         // debug tint off: mul == 1 and decode -> x1 -> encode is the identity on all 256 (1024, 4) codes (exhaustive
         // check in tests/test_host_logic.py), so the texel bits are copied straight from the TMA landing zone
-        const uint32_t *q = sRaw + (y0 - sy0) * kRcasRawW + (x - sx0) + 3;
+        const uint32_t *q = sRaw + (y0 - sy0) * kRcasRawW + (x - sx0) + a.boxShift;
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
           const int y = y0 + k;

@@ -8,7 +8,15 @@
 
 namespace ovrfsr {
 
-struct PassImage { void *ptr; uint32_t pitch; int w, h; int format; };
+// ptr/pitch/w/h: the image a pass reads or writes.  It may be a rectangle of a larger texture (ovrfsr_apply_bounds):
+// ptr then points at the rectangle's texel (x0, y0) of a texture texW x texH texels large.  texW == 0: the image is
+// the whole texture.  The kernels treat the rectangle's edge as the texture's edge; TMA descriptors stay keyed by
+// the whole texture, so a rectangle that changes every frame keeps hitting the descriptor cache.
+struct PassImage {
+  void *ptr; uint32_t pitch; int w, h; int format;
+  int x0 = 0, y0 = 0, texW = 0, texH = 0;
+  bool is_crop() const { return texW != 0 && (x0 != 0 || y0 != 0 || w != texW || h != texH); }
+};
 
 // FSR (fsr_kernels.cuh).  consts are the reference's constant-buffer layouts.
 // `direct` (EASU) / `skipOutside` (RCAS) are the ctx path's pairing of the two passes: when RCAS follows EASU in the same
@@ -35,6 +43,10 @@ cudaError_t launch_nis_scaler_fast(const PassImage &src, const PassImage &dst, c
 cudaError_t launch_nis_scaler_strict(const PassImage &src, const PassImage &dst, const void *cfg256, const float *coef, cudaStream_t s);
 cudaError_t launch_nis_sharpen_fast(const PassImage &src, const PassImage &dst, const void *cfg256, const float *coef, cudaStream_t s);
 cudaError_t launch_nis_sharpen_strict(const PassImage &src, const PassImage &dst, const void *cfg256, const float *coef, cudaStream_t s);
+
+// NVScaler (sharpen == false) or NVSharpen in the given math mode: what ovrfsr_dispatch_nis_scaler / _sharpen run on
+// their checked images, and the ctx path's NIS passes (nis_capi.cu)
+cudaError_t launch_nis(bool sharpen, const PassImage &src, const PassImage &dst, const void *cfg256, int math_mode, cudaStream_t s);
 
 // legacy CAS (cas_kernels.cuh).  consts = const0, const1 of src/cas/cas.compute.h:1-4 as CasSetup fills them.
 cudaError_t launch_cas_fast(const PassImage &src, const PassImage &dst, const uint32_t consts[8], int sharpenOnly, cudaStream_t s);

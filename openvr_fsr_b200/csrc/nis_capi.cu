@@ -54,6 +54,16 @@ int status_of(cudaError_t e) {
 }
 } // namespace
 
+cudaError_t ovrfsr::launch_nis(bool sharpen, const PassImage &src, const PassImage &dst, const void *cfg256, int math_mode,
+                               cudaStream_t s) {
+  static float both[2][64 * 8];
+  static std::once_flag once;
+  std::call_once(once, [&] { std::memcpy(both[0], ovrfsr_nis_coef_scale(), sizeof(both[0])); std::memcpy(both[1], ovrfsr_nis_coef_usm(), sizeof(both[1])); });
+  const bool strict = math_mode == OVRFSR_MATH_STRICT;
+  if (sharpen) return strict ? launch_nis_sharpen_strict(src, dst, cfg256, nullptr, s) : launch_nis_sharpen_fast(src, dst, cfg256, nullptr, s);
+  return strict ? launch_nis_scaler_strict(src, dst, cfg256, &both[0][0], s) : launch_nis_scaler_fast(src, dst, cfg256, &both[0][0], s);
+}
+
 extern "C" {
 
 int ovrfsr_dispatch_nis_scaler(const ovrfsr_image *src, const ovrfsr_image *dst, const void *cfg256, int math_mode,
@@ -63,13 +73,7 @@ int ovrfsr_dispatch_nis_scaler(const ovrfsr_image *src, const ovrfsr_image *dst,
   if (!cfg256) return OVRFSR_ERR_INVALID;
   int rc = check(src, false);
   if (rc != OVRFSR_OK || (rc = check(dst, true)) != OVRFSR_OK) return rc;
-  const float *coef = ovrfsr_nis_coef_scale(); // g_coefScale and g_coefUsm are contiguous? no: upload buffer below
-  static float both[2][64 * 8];
-  static std::once_flag once;
-  std::call_once(once, [&] { std::memcpy(both[0], coef, sizeof(both[0])); std::memcpy(both[1], ovrfsr_nis_coef_usm(), sizeof(both[1])); });
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  return status_of(math_mode == OVRFSR_MATH_STRICT ? launch_nis_scaler_strict(pass(*src), pass(*dst), cfg256, &both[0][0], s)
-                                                   : launch_nis_scaler_fast(pass(*src), pass(*dst), cfg256, &both[0][0], s));
+  return status_of(launch_nis(false, pass(*src), pass(*dst), cfg256, math_mode, static_cast<cudaStream_t>(stream)));
 }
 
 int ovrfsr_dispatch_nis_sharpen(const ovrfsr_image *src, const ovrfsr_image *dst, const void *cfg256, int math_mode,
@@ -80,9 +84,7 @@ int ovrfsr_dispatch_nis_sharpen(const ovrfsr_image *src, const ovrfsr_image *dst
   int rc = check(src, false);
   if (rc != OVRFSR_OK || (rc = check(dst, true)) != OVRFSR_OK) return rc;
   if (src->width != dst->width || src->height != dst->height) return OVRFSR_ERR_INVALID;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  return status_of(math_mode == OVRFSR_MATH_STRICT ? launch_nis_sharpen_strict(pass(*src), pass(*dst), cfg256, nullptr, s)
-                                                   : launch_nis_sharpen_fast(pass(*src), pass(*dst), cfg256, nullptr, s));
+  return status_of(launch_nis(true, pass(*src), pass(*dst), cfg256, math_mode, static_cast<cudaStream_t>(stream)));
 }
 
 } // extern "C"

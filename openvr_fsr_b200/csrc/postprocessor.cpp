@@ -78,7 +78,14 @@ void PostProcessor::Apply(EVREye eEye, const Texture_t *pTexture, const VRTextur
   const int onlyOneEye = std::abs(pBounds->uMax - pBounds->uMin) > .5f;
   const int eye = eEye == Eye_Right ? 1 : 0;
   ovrfsr_image out{};
-  const int rc = ovrfsr_apply(ctx, eye, texture, onlyOneEye, &out, stream);
+  int rc;
+  if (Config::Instance().honourTextureBounds) {
+    // the bounds go on to the real Submit untouched: the output rectangle sits where they point
+    const ovrfsr_bounds b{pBounds->uMin, pBounds->vMin, pBounds->uMax, pBounds->vMax};
+    rc = ovrfsr_apply_bounds(ctx, eye, texture, &b, &out, nullptr, stream);
+  } else {
+    rc = ovrfsr_apply(ctx, eye, texture, onlyOneEye, &out, stream);
+  }
   if (rc == OVRFSR_PASSTHROUGH) {
     return;
   }
